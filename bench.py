@@ -59,6 +59,8 @@ def parse():
     ap.add_argument("--only", default="", help="comma list of extra blocks to run (t480,beam,train,gpu_reference,transformer); default: all")
     ap.add_argument("--no-gpu-reference-tfm", action="store_true", help="skip the eager-PyTorch timing inside the transformer block")
     ap.add_argument("--train-steps", type=int, default=3)
+    ap.add_argument("--dump-outputs", metavar="DIR", default="",
+                    help="write the outputs of the headline's last timed step (rank 0) as .npy files under DIR")
     return ap.parse_args()
 
 
@@ -211,8 +213,8 @@ def measure_decode(ctx, args, T, full):
     pin = {k: inp[k].pin_memory() for k in KEYS}
 
     def step_dev():
-        nm.prologue(*(dev[k] for k in KEYS), want_sim=True)
-        return nm.decode_greedy(B, T, dev["pnt_mask"])
+        sim = nm.prologue(*(dev[k] for k in KEYS), want_sim=True)
+        return nm.decode_greedy(B, T, dev["pnt_mask"]) + (sim,)
 
     for _ in range(W):
         step_dev()
@@ -221,9 +223,10 @@ def measure_decode(ctx, args, T, full):
     if ctx.rank == 0 and full and not args.quick:
         sampler.start()
     l0 = capi.kernel_launches()
-    ms, (seq, logp, att2) = ctx.timed(step_dev, K)
+    ms, (seq, logp, att2, sim) = ctx.timed(step_dev, K)
     launches = capi.kernel_launches() - l0
-    r = dict(opt=opt, sd=sd, ms=ms, launches=launches, uniq=int(len(torch.unique(seq))), B=B, K=K, W=W, T=T)
+    r = dict(opt=opt, sd=sd, ms=ms, launches=launches, uniq=int(len(torch.unique(seq))), B=B, K=K, W=W, T=T,
+             outputs=dict(seq=seq, logp=logp, att2=att2, sim=sim))
     if args.quick:
         r["clocks"] = None
         return r
@@ -246,7 +249,7 @@ def measure_decode(ctx, args, T, full):
         capi.profile_enable(True)
         ctx.barrier()
         for _ in range(K):
-            seq_p, _, _ = step_dev()
+            seq_p = step_dev()[0]
         ctx.barrier()
         capi.profile_enable(False)
         r["stages"] = capi.profile_read()
@@ -471,11 +474,34 @@ def gpu_reference(opt, sd, B, T):
             "(fp32, allow_tf32=False, cudnn.benchmark=True), eager", "torch": torch.__version__}
 
 
+DUMP_BYTES = 63_000_000                     # array bytes of --dump-outputs; the .npy headers stay within the rest of 64 MB
+
+
+def dump_outputs(path, seq, logp, att2, sim):
+    """--dump-outputs: what one headline step hands its caller, as .npy files, so that two builds run with the same arguments (hence the
+    same seeded inputs) can be compared output for output.  seq (token ids, as exact float64) and logp are written whole; att2 and sim
+    (1.8 MB per clip at the default sizes) on a fixed, seeded sample of clips, listed in clips.npy, that keeps the directory under 64 MB."""
+    import numpy as np
+    os.makedirs(path, exist_ok=True)
+    B = seq.shape[0]
+    out = {"seq": seq.double(), "logp": logp.float()}
+    room = DUMP_BYTES - sum(t.numel() * t.element_size() for t in out.values()) - B * 8
+    n = min(B, room // ((att2[0].numel() + sim[0].numel()) * 4))
+    clips = torch.randperm(B, generator=torch.Generator().manual_seed(0))[:n].sort().values
+    out.update(clips=clips.double(), att2=att2[clips.to(att2.device)], sim=sim[clips.to(sim.device)])
+    for name, t in out.items():
+        np.save(os.path.join(path, name + ".npy"), t.cpu().numpy())
+
+
 def run_ours(args):
     ctx = Ctx(args)
     only = set(x for x in args.only.split(",") if x) or {"t480", "beam", "train", "gpu_reference", "transformer"}
     T = args.frames
     r = measure_decode(ctx, args, T, True)
+    outputs = r.pop("outputs")
+    if args.dump_outputs and ctx.rank == 0:
+        dump_outputs(args.dump_outputs, **outputs)
+    del outputs
     opt, B, K, W = r["opt"], r["B"], r["K"], r["W"]
     world = ctx.world
     tokens = world * B * opt.seq_length * K
