@@ -34,7 +34,9 @@ extern "C" GVD_API int gvd_op_kernel_launches(void) { return (int)g_launches.loa
 // kernel (measured: no gain, off); bit 6 (64) programmatic dependent launch in the decode loop (measured: no gain, off); bit 7 (128)
 // conversion-free persistent GEMMs for the prologue (activations packed into the fp16x3 image, both operands straight from TMA); bit 8 (256)
 // fp16x3 images instead of tf32 planes in the fused self-attention pair; bit 9 (512) pack fusion: the producer of a prologue activation (GEMM
-// epilogue / row kernel) stores the fp16x3 operand image the next GEMM streams, instead of a separate pack pass.
+// epilogue / row kernel) stores the fp16x3 operand image the next GEMM streams, instead of a separate pack pass; bit 10 (1024) CTA pairs in
+// the persistent prologue GEMM (measured slower: off); bit 11 (2048) thread-per-row epilogue stores in the persistent prologue GEMM (the
+// reference its staged epilogue is tested against).
 // Default 923 = 1 + 2 + 8 + 16 + 128 + 256 + 512.
 static std::atomic<int> g_backend{923};
 int gvd_backend() { return g_backend.load(std::memory_order_relaxed); }

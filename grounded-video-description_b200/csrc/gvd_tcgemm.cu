@@ -2260,15 +2260,96 @@ __device__ __forceinline__ void ss_store_row(const SsParams& p, const float (&ac
     }
 }
 
+// Warp-private staging tiles of the persistent kernels' epilogue (ss_store_staged): one 32 x 32 fp32 tile per drain warp, placed after the
+// barriers, outside the TMA ring (which keeps streaming the next tile while the epilogue runs).
+constexpr int SS_STG_OFF = 256, SS_STG_BYTES = 8 * 32 * 128;
+template <class Cfg> constexpr size_t ss_persist_smem() {
+    static_assert(8 * (2 * Cfg::NST + 4) + 4 <= SS_STG_OFF && Cfg::DRAIN_WARPS * 32 * 128 <= SS_STG_BYTES, "staging tiles after the barriers");
+    static_assert(Cfg::SMEM + SS_STG_OFF + SS_STG_BYTES <= 227 * 1024, "ring + staging exceed the 227 KB of shared memory a block may use");
+    return Cfg::SMEM + SS_STG_OFF + SS_STG_BYTES;
+}
+
+// The plain-mode epilogue of ss_store_row (same values, same destinations) as coalesced stores: a drain warp owns rows [mrow0, mrow0 + 32) x
+// columns [ncol0, ncol0 + ACC) (lane <-> row).  Per 32-column block, phase 1: each thread writes its row's accumulators into the warp's 4 KB
+// staging tile `stg`, 16-byte chunks XOR-swizzled by the row so that the row-wise writes and the 4-rows-per-instruction reads are both free
+// of bank conflicts; phase 2: lane = (row lane / 8 + 4 i, chunk lane % 8) applies bias / activation to its 4 columns and stores them, so 8
+// consecutive lanes store one row's 128 bytes of C, or the 64-byte hi and lo halves of its image K slice (a 32-column block is exactly one
+// K slice), instead of every store instruction touching 32 lines.
+template <int ACC>
+__device__ __forceinline__ void ss_store_staged(const SsParams& p, const float (&acc)[ACC], const int mrow0, const int ncol0, const int lane, const bool vec_ok,
+                                                const uint32_t stg) {
+    const int c = lane & 7;
+#pragma unroll
+    for (int jb = 0; jb < ACC; jb += 32) {
+        const int nb = ncol0 + jb;                    // (warp-uniform)
+        if (nb >= p.N) break;
+#pragma unroll
+        for (int j = 0; j < 32; j += 4)
+            sts128(stg + (uint32_t)lane * 128u + (uint32_t)(((j >> 2) ^ (lane & 7)) << 4),
+                   make_float4(acc[jb + j], acc[jb + j + 1], acc[jb + j + 2], acc[jb + j + 3]));
+        __syncwarp();
+        // a lane keeps its 4 columns for the whole block: bias / affine loaded once (the row-owning thread would load all 32)
+        const int n = nb + 4 * c;
+        float bv[4], sv[4], hv[4];
+#pragma unroll
+        for (int e = 0; e < 4; ++e) {
+            const bool ok = n + e < p.N;
+            bv[e] = (ok && p.bias) ? __ldg(p.bias + n + e) : 0.f;
+            sv[e] = (ok && p.act == GVD_ACT_RELU_AFFINE_RELU) ? __ldg(p.scale2 + n + e) : 0.f;
+            hv[e] = (ok && p.act == GVD_ACT_RELU_AFFINE_RELU) ? __ldg(p.shift2 + n + e) : 0.f;
+        }
+#pragma unroll
+        for (int i = 0; i < 8; ++i) {
+            const int rr = i * 4 + (lane >> 3);
+            const float4 t = lds128(stg + (uint32_t)rr * 128u + (uint32_t)((c ^ (rr & 7)) << 4));
+            const int m = mrow0 + rr;
+            if (m >= p.M) continue;
+            float v[4] = {t.x, t.y, t.z, t.w};
+#pragma unroll
+            for (int e = 0; e < 4; ++e) {             // the operations of ss_store_row, element by element
+                float x = v[e];
+                if (n + e < p.N) {
+                    if (p.bias) x += bv[e];
+                    if (p.act >= GVD_ACT_RELU) x = fmaxf(x, 0.f);
+                    if (p.act == GVD_ACT_RELU_AFFINE_RELU) x = fmaxf(fmaf(x, sv[e], hv[e]), 0.f);
+                } else {
+                    x = 0.f;                          // padding columns of the image are zeros
+                }
+                v[e] = x;
+            }
+            if (p.C) {
+                float* d = p.C + (long long)m * p.ldc + n;
+                if (vec_ok && n + 3 < p.N) {
+                    *reinterpret_cast<float4*>(d) = make_float4(v[0], v[1], v[2], v[3]);
+                } else {
+#pragma unroll
+                    for (int e = 0; e < 4; ++e)
+                        if (n + e < p.N) d[e] = v[e];
+                }
+            }
+            if (p.img && n < p.ld_img) {
+                uint32_t h0, l0, h1, l1;
+                f16x3_split_pair(v[0], v[1], p.img_scale, h0, l0);
+                f16x3_split_pair(v[2], v[3], p.img_scale, h1, l1);
+                uint32_t* w = p.img + (long long)m * p.ld_img + f16x3_word(n);
+                *reinterpret_cast<uint2*>(w) = make_uint2(h0, h1);
+                *reinterpret_cast<uint2*>(w + 16) = make_uint2(l0, l1);
+            }
+        }
+        __syncwarp();                                 // the next block's phase 1 overwrites the tile
+    }
+}
+
 // =====================================================================================================
 // f16ss_persistent_kernel — f16ss_kernel (EPI 0) as a persistent tile loop: one CTA per SM walks the output tiles (N tiles of one M row
 // block consecutively, so the A row block stays in L2), the TMA producer and the MMA issuer run ahead into the next tile while the drain
 // warps finish the previous one: the per-CTA set-up (barriers, TMEM allocation, descriptor fetch), the pipeline fill and the epilogue
-// no longer sit between two tiles' MMAs (they were ~30 % of a 32-slice tile).  The epilogue writes its rows straight from registers
-// (each thread owns one output row x BN/2 columns: 16-byte stores, whole 32-byte sectors), so no pipeline buffer is borrowed for
-// staging and the ring keeps streaming.
+// no longer sit between two tiles' MMAs (they were ~30 % of a 32-slice tile).  Each drain thread owns one output row x BN/2 columns; the
+// plain-mode epilogue (ss_store_staged) goes out through a warp-private staging tile outside the ring, so the ring keeps streaming and the
+// stores leave as whole 128-byte lines.  ROWS: thread-per-row stores from registers (ss_store_row: the Q|K|V mode, and the reference the
+// staged epilogue is tested against); a separate instantiation, because one kernel holding both epilogues spilled more and ran slower.
 // =====================================================================================================
-template <int BN>
+template <int BN, bool ROWS>
 __global__ void __launch_bounds__(SsCfg<BN, 0>::THREADS, 1)
 f16ss_persistent_kernel(const __grid_constant__ CUtensorMap mapA, const __grid_constant__ CUtensorMap mapB, const SsParams p, int tiles_n, int tiles_total) {
     using Cfg = SsCfg<BN, 0>;
@@ -2354,6 +2435,7 @@ f16ss_persistent_kernel(const __grid_constant__ CUtensorMap mapA, const __grid_c
         const int cbeg = (dw >> 2) * ACC;
         const int row = q * 32 + lane;
         const bool vec_ok = (p.ldc % 4 == 0) && ((reinterpret_cast<uintptr_t>(p.C) & 15) == 0);
+        const uint32_t stg = smem_u32(smem + (size_t)NST * Cfg::STAGE + SS_STG_OFF) + (uint32_t)dw * 4096u;
         int c = 0;
         for (int tile = blockIdx.x; tile < tiles_total; tile += gridDim.x) {
             const int m0 = (tile / tiles_n) * TC_BM, n0 = (tile % tiles_n) * BN;
@@ -2374,7 +2456,8 @@ f16ss_persistent_kernel(const __grid_constant__ CUtensorMap mapA, const __grid_c
 #pragma unroll
                 for (int e = 0; e < ACC; ++e) acc[e] = fmaf(__uint_as_float(r[e]), p.oscale, acc[e]);
             }
-            ss_store_row<ACC>(p, acc, m0 + row, n0 + cbeg, lane, vec_ok);
+            if constexpr (ROWS) ss_store_row<ACC>(p, acc, m0 + row, n0 + cbeg, lane, vec_ok);
+            else ss_store_staged<ACC>(p, acc, m0 + q * 32, n0 + cbeg, lane, vec_ok, stg);
         }
     }
     asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
@@ -2420,6 +2503,7 @@ __device__ __forceinline__ void umma_commit_pair_elect(uint64_t* bar) {         
         "}\n" ::"r"(smem_u32(bar))
         : "memory");
 }
+template <bool ROWS>
 __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(PairCfg::THREADS, 1)
 f16ss_pair_kernel(const __grid_constant__ CUtensorMap mapA, const __grid_constant__ CUtensorMap mapB, const SsParams p, int tiles_n, int tiles_total) {
     using Cfg = PairCfg;
@@ -2514,6 +2598,7 @@ f16ss_pair_kernel(const __grid_constant__ CUtensorMap mapA, const __grid_constan
         const int cbeg = (dw >> 2) * ACC;
         const int row = q * 32 + lane;
         const bool vec_ok = (p.ldc % 4 == 0) && ((reinterpret_cast<uintptr_t>(p.C) & 15) == 0);
+        const uint32_t stg = smem_u32(smem + (size_t)NST * Cfg::STAGE + SS_STG_OFF) + (uint32_t)dw * 4096u;
         int c = 0;
         for (int tile = pair; tile < tiles_total; tile += npairs) {
             const int m0 = (tile / tiles_n) * 256 + (int)rank * TC_BM, n0 = (tile % tiles_n) * 256;
@@ -2534,7 +2619,8 @@ f16ss_pair_kernel(const __grid_constant__ CUtensorMap mapA, const __grid_constan
 #pragma unroll
                 for (int e = 0; e < ACC; ++e) acc[e] = fmaf(__uint_as_float(r[e]), p.oscale, acc[e]);
             }
-            ss_store_row<ACC>(p, acc, m0 + row, n0 + cbeg, lane, vec_ok);
+            if constexpr (ROWS) ss_store_row<ACC>(p, acc, m0 + row, n0 + cbeg, lane, vec_ok);
+            else ss_store_staged<ACC>(p, acc, m0 + q * 32, n0 + cbeg, lane, vec_ok, stg);
         }
     }
     asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
@@ -2794,6 +2880,16 @@ int gvd_gru_layer_f16(const float* gi, const float* Whh_img, const float* bhh, f
 static thread_local int g_sm_reserve = 0;
 int gvd_sm_reserve(int n) { const int old = g_sm_reserve; g_sm_reserve = n < 0 ? 0 : n; return old; }
 
+using SsPersistentFn = void (*)(CUtensorMap, CUtensorMap, SsParams, int, int);
+template <SsPersistentFn F>
+static int launch_ss_persistent(size_t smem, int ctas, int threads, const CUtensorMap& mA, const CUtensorMap& mB, const SsParams& p, int tiles_n, int tiles,
+                                cudaStream_t st) {
+    static bool a = false;
+    if (!a) { GVD_CHECK_CUDA(cudaFuncSetAttribute(F, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem)); a = true; }
+    F<<<ctas, threads, smem, st>>>(mA, mB, p, tiles_n, tiles);
+    return 0;
+}
+
 // C[M, N] = act(A W^T + bias) with both operands in the fp16x3 image: Ap [M, lda] words (scale GVD_F16_SA), Wp [N, ldw] words (scale
 // GVD_F16_SW), lda / ldw multiples of 32 covering K rounded up to 32 (zero padded)
 int gvd_gemm_f16ss(const float* Ap, long long lda, const float* Wp, long long ldw, const float* bias, const float* scale2, const float* shift2, int act,
@@ -2843,28 +2939,27 @@ int gvd_gemm_f16ss(const float* Ap, long long lda, const float* Wp, long long ld
         // SMs left free for a concurrent stream (the bi-GRU chain of the frame branch: gvd_sm_reserve, set by the prologue around the region stages)
         const int ctas = (int)std::min<long long>(tiles, std::max(1, sms - g_sm_reserve));
         static const bool no_pair = getenv("GVD_SS_NO_PAIR") != nullptr;
+        // thread-per-row epilogue stores (ss_store_row) for the Q|K|V projection (staged, its per-head routing measured slower: interact.qkv_proj
+        // 5.6 vs 4.8 ms per step) and under backend bit 11, the reference the staged epilogue is tested against
+        const bool rows = qkv || (gvd_backend() & 2048) != 0;
         if (bn == 256 && !no_pair && (gvd_backend() & 1024) != 0 && sms % 2 == 0) {
             // CTA pairs (backend bit 10): 256 x 256 tiles, each CTA streams half of the B tile
             CUtensorMap mB2;
             GVD_TRY(make_map(&mB2, Wp, Kp, N, ldw, 1, 0, 1, 0, 128, &d0, &d1));
-            static bool a = false;
-            if (!a) { GVD_CHECK_CUDA(cudaFuncSetAttribute(f16ss_pair_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)PairCfg::SMEM)); a = true; }
             const int tn2 = gvd_cdiv(N, 256);
             const long long tiles2 = (long long)tn2 * gvd_cdiv(M, 256);
             const int ctas2 = (int)std::min<long long>(2 * tiles2, std::max(2, (sms - g_sm_reserve) & ~1));
-            f16ss_pair_kernel<<<ctas2, PairCfg::THREADS, PairCfg::SMEM, st>>>(mA, mB2, p, tn2, (int)tiles2);
+            GVD_TRY((rows ? launch_ss_persistent<f16ss_pair_kernel<true>> : launch_ss_persistent<f16ss_pair_kernel<false>>)(
+                ss_persist_smem<PairCfg>(), ctas2, PairCfg::THREADS, mA, mB2, p, tn2, (int)tiles2, st));
         } else if (bn == 256) {
-            static bool a = false;
-            if (!a) { GVD_CHECK_CUDA(cudaFuncSetAttribute(f16ss_persistent_kernel<256>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)SsCfg<256, 0>::SMEM)); a = true; }
-            f16ss_persistent_kernel<256><<<ctas, SsCfg<256, 0>::THREADS, SsCfg<256, 0>::SMEM, st>>>(mA, mB, p, tiles_n, (int)tiles);
+            GVD_TRY((rows ? launch_ss_persistent<f16ss_persistent_kernel<256, true>> : launch_ss_persistent<f16ss_persistent_kernel<256, false>>)(
+                ss_persist_smem<SsCfg<256, 0>>(), ctas, SsCfg<256, 0>::THREADS, mA, mB, p, tiles_n, (int)tiles, st));
         } else if (bn == 128) {
-            static bool a = false;
-            if (!a) { GVD_CHECK_CUDA(cudaFuncSetAttribute(f16ss_persistent_kernel<128>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)SsCfg<128, 0>::SMEM)); a = true; }
-            f16ss_persistent_kernel<128><<<ctas, SsCfg<128, 0>::THREADS, SsCfg<128, 0>::SMEM, st>>>(mA, mB, p, tiles_n, (int)tiles);
+            GVD_TRY((rows ? launch_ss_persistent<f16ss_persistent_kernel<128, true>> : launch_ss_persistent<f16ss_persistent_kernel<128, false>>)(
+                ss_persist_smem<SsCfg<128, 0>>(), ctas, SsCfg<128, 0>::THREADS, mA, mB, p, tiles_n, (int)tiles, st));
         } else {
-            static bool a = false;
-            if (!a) { GVD_CHECK_CUDA(cudaFuncSetAttribute(f16ss_persistent_kernel<64>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)SsCfg<64, 0>::SMEM)); a = true; }
-            f16ss_persistent_kernel<64><<<ctas, SsCfg<64, 0>::THREADS, SsCfg<64, 0>::SMEM, st>>>(mA, mB, p, tiles_n, (int)tiles);
+            GVD_TRY((rows ? launch_ss_persistent<f16ss_persistent_kernel<64, true>> : launch_ss_persistent<f16ss_persistent_kernel<64, false>>)(
+                ss_persist_smem<SsCfg<64, 0>>(), ctas, SsCfg<64, 0>::THREADS, mA, mB, p, tiles_n, (int)tiles, st));
         }
         GVD_CHECK_LAUNCH();
         return 0;
